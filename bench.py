@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (headline workload)
   python bench.py --impl reference --gpus N --steps K ...  # the reference's own CPU path (oracle/_ref, else the oracle port)
   python bench.py --workload {sigmoid_cora,layer,segmented,fwdbwd}   # the other SURVEY 8 rows, one JSON line each (1 GPU)
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # also write what the last timed step computed, DIR/out.npy
 
 Headline workload ("simple")
   step      = one `full_attention_conv(q, k, v, 'simple')` forward (pass 1 reduce -> [all-reduce] -> pass 2 apply) over
@@ -26,6 +27,7 @@ import os
 import sys
 import time
 
+sys.dont_write_bytecode = True      # the tree may be read-only, and a run leaves nothing in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -303,18 +305,32 @@ class Problem:
 
 
 def timed(fn, steps, barrier, dev, group):
+    """-> (ms per step, what the last of the `steps` timed calls of fn returned)"""
     import torch.distributed as dist
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
     barrier()
     ev[0].record()
-    for _ in range(steps):
+    for _ in range(steps - 1):
         fn()
+    last = fn()
     ev[1].record()
     barrier()
     t = torch.tensor([ev[0].elapsed_time(ev[1]) / steps], dtype=torch.float64, device=dev)
     if group is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX, group=group)
-    return float(t.item())
+    return float(t.item()), last
+
+
+DUMP_ROWS = 32768       # rows of the [N, H, D] output --dump-outputs keeps (32 MiB in fp32)
+
+
+def dump_outputs(out_dir, out):
+    """Writes out_dir/out.npy: a fixed sample (DUMP_ROWS rows drawn once with seed 0, in ascending order) of `out`, the [N, H, D]
+    result of the last timed step, in float32.  The same arguments give the same inputs, so two builds compare output for output."""
+    import numpy as np
+    rows = torch.randperm(out.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "out.npy"), out.index_select(0, rows.to(out.device)).float().cpu().numpy())
 
 
 def run_ours(args):
@@ -375,9 +391,12 @@ def run_ours(args):
     sampler = ClockSampler(dev)
     barrier()
     sampler.begin()
-    ms = timed(prob.step, args.steps, barrier, dev, group)
+    ms, out = timed(prob.step, args.steps, barrier, dev, group)
     sampler.end()
     value = N_NODES * world / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
+    del out
 
     # ---- cold-cache number (SURVEY 8d): L2 flushed (256 MB written) before every step, each step timed on its own
     cold_ms = None
@@ -469,7 +488,7 @@ def run_ours(args):
         par_b = pb.parity(dev)
         for _ in range(3):
             pb.step()
-        ms_b = timed(pb.step, max(5, min(args.steps, 20)), barrier, dev, group)
+        ms_b, _ = timed(pb.step, max(5, min(args.steps, 20)), barrier, dev, group)
         cfg_b = {"workload": f"full_attention_conv('simple') N={N_CFG_B} H={HEADS} D={DIM} fp32 row-sharded over {world} GPU(s) (BASELINE configs[3])",
                  "scaling": "strong", "rows_this_rank": b1 - b0, "ms_per_step": ms_b, "value": N_CFG_B / (ms_b * 1e-3), "unit": UNIT,
                  "roofline_frac": 4 * N_CFG_B * HEADS * DIM * 4 / (ms_b * 1e-3) / 1e9 / (measured_peaks()[0] * world), "parity": par_b}
@@ -496,7 +515,7 @@ def run_ours(args):
             del wp, want
             for _ in range(5):
                 ops.simple_forward(qb, kb, vb)
-            ms16 = timed(lambda: ops.simple_forward(qb, kb, vb), args.steps, barrier, dev, None)
+            ms16, _ = timed(lambda: ops.simple_forward(qb, kb, vb), args.steps, barrier, dev, None)
             lp16 = {"dtype": "bf16", "ms_per_step": ms16, "value": N_NODES / (ms16 * 1e-3), "unit": UNIT,
                     "roofline": {"bound": "hbm", "achieved": 2 * T / (ms16 * 1e-3) / 1e9, "peak": measured_peaks()[0], "unit": "GB/s",
                                  "frac": 2 * T / (ms16 * 1e-3) / 1e9 / measured_peaks()[0], "algorithmic_bytes_per_step": 2 * T},
@@ -787,7 +806,14 @@ def main():
     ap.add_argument("--layer-gcn", default="spmm", choices=["spmm", "epilogue"], help="--workload layer: where the gcn term is computed")
     ap.add_argument("--no-cfg-b", action="store_true", help="skip the BASELINE configs[3] (N=1.6M strong-scaling) leg")
     ap.add_argument("--collective", default="nvlink", choices=["nvlink", "nccl"], help="multi-GPU all-reduce of the partials")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help=f"headline workload: after the timed steps write DIR/out.npy, {DUMP_ROWS} fixed rows (seed 0) of the [N, H, D] fp32 "
+                         "output of the last timed step (rank 0's rows with several GPUs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "simple"):
+        ap.error("--dump-outputs covers the headline workload (--impl ours --workload simple)")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload != "simple":

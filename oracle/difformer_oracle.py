@@ -10,8 +10,7 @@ Pinning: the reference ships no tests or golden vectors (SURVEY.md section 4/8c)
 pinned against the reference *itself*: `oracle/make_golden.py` runs the unmodified reference
 files (under `oracle/ref_shim.py`) in the build container and commits input/output vectors to
 `tests/golden/`; `tests/test_oracle_golden.py` checks every function below against those
-vectors, and the last test there re-runs the live reference when /root/reference
-is present.  All line citations are relative to /root/reference/.
+vectors.  All line citations are relative to the root of the reference project.
 
 Algebra is written in matmul/reduction form on purpose (the reference uses einsum chains and
 materialises broadcasts) so agreement is a meaningful check of the algorithm, not of a copy.

@@ -12,8 +12,8 @@ installable in this image (no wheel, no network):
 
 This file injects minimal stand-ins for exactly those three names (documented semantics of the
 pinned versions) so the reference files import *unmodified*.  It is used by
-`oracle/make_golden.py` (fixture generation), by CPU tests that pin the restatement in
-`oracle/difformer_oracle.py` against the real reference, and by `bench.py`'s CPU-baseline leg
+`oracle/make_golden.py` (fixture generation: the tests pin the restatement in
+`oracle/difformer_oracle.py` against those recorded reference outputs) and by `bench.py`'s CPU-baseline leg
 (the reference's own `full_attention_conv` timed on the host cores).  The product path never
 imports it.
 """

@@ -114,47 +114,25 @@ def test_epilogue_struct_layout():
 
 def test_reference_parse_method_builds_this_model():
     """SURVEY 8b: the harness builds the model through `parse.parse_method` after `from difformer import *` (node
-    classification/parse.py:2-10).  Run the reference's own, unmodified parse.py with this repo's `difformer` module on the
-    import path: the object it returns must be this drop-in, with exactly the reference model's parameter names and shapes."""
-    import argparse
-    import importlib.util
+    classification/parse.py:2-10).  Replay the DIFFormer(...) calls the reference's own, unmodified parse.py makes on two command
+    lines (recorded by oracle/make_golden.py, group parse_method) against this repo's `difformer` module: the object built must be
+    this drop-in, with exactly the reference model's parameter names and shapes."""
+    import json
     import os
-    import sys
-    import types
-    path = "/root/reference/node classification/parse.py"
-    if not os.path.isfile(path):
-        pytest.skip("reference harness not present")
-    from oracle.ref_shim import load_reference_v1
-    saved = {k: sys.modules.get(k) for k in ("gnns", "difformer")}
-    sys.modules["gnns"] = types.ModuleType("gnns")          # baseline GNN zoo (PyG): out of scope, star-import of an empty module
-    sys.modules["difformer"] = difformer
-    try:
-        spec = importlib.util.spec_from_file_location("_reference_parse", path)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        parser = argparse.ArgumentParser()
-        mod.parser_add_main_args(parser)
-        for argv in (["--use_bn", "--use_residual", "--use_graph", "--hidden_channels", "64"],
-                     ["--use_bn", "--use_residual", "--use_graph", "--use_weight", "--use_source", "--num_heads", "4", "--kernel", "sigmoid",
-                      "--hidden_channels", "32", "--num_layers", "3", "--graph_weight", "0.5"]):
-            args = parser.parse_args(argv)
-            model = mod.parse_method(args, 100, 7, 33, torch.device("cpu"))
-            assert type(model) is difformer.DIFFormer
-            ref = load_reference_v1().DIFFormer(33, args.hidden_channels, 7, num_layers=args.num_layers, alpha=args.alpha, dropout=args.dropout,
-                                                num_heads=args.num_heads, kernel=args.kernel, use_bn=args.use_bn, use_residual=args.use_residual,
-                                                use_graph=args.use_graph, use_weight=args.use_weight, use_source=args.use_source,
-                                                graph_weight=args.graph_weight)
-            got = {k: tuple(v.shape) for k, v in model.state_dict().items()}
-            want = {k: tuple(v.shape) for k, v in ref.state_dict().items()}
-            assert got == want
-            model.load_state_dict(ref.state_dict())           # checkpoints round-trip (test_large_dataset.py:86-88)
-            model.reset_parameters()                           # main.py:110
-    finally:
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
+    from tests.conftest import GOLDEN
+    with open(os.path.join(GOLDEN, "parse_method.json")) as f:
+        calls = json.load(f)
+    assert len(calls) == 2
+    for argv, call in calls.items():
+        model = difformer.DIFFormer(*call["args"], **call["kwargs"]).to(torch.device("cpu"))
+        assert type(model) is difformer.DIFFormer, argv
+        got = {k: list(v.shape) for k, v in model.state_dict().items()}
+        assert got == call["state_dict_shapes"], argv
+        gen = torch.Generator().manual_seed(0)
+        ref_sd = {k: torch.randn(shape, generator=gen) for k, shape in call["state_dict_shapes"].items()}
+        model.load_state_dict(ref_sd)                      # checkpoints round-trip (test_large_dataset.py:86-88)
+        assert all(torch.equal(model.state_dict()[k], t) for k, t in ref_sd.items())
+        model.reset_parameters()                           # main.py:110
 
 
 @pytest.mark.parametrize("h,use_weight", [(1, True), (2, False), (4, True)])

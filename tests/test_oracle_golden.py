@@ -1,20 +1,29 @@
 """CPU: pins oracle/difformer_oracle.py against the committed reference outputs (tests/golden,
-made by oracle/make_golden.py from the unmodified reference) and, when /root/reference is
-present, against the live reference.  Tolerances: 1e-5 rel in fp32 (pure reassociation noise),
+made by oracle/make_golden.py from the unmodified reference).  Tolerances: 1e-5 rel in fp32 (pure reassociation noise),
 2e-6 when the oracle runs in fp64 on the fp32 inputs."""
-import os
+import filecmp
+import json
 
 import pytest
 import torch
 
 from oracle import difformer_oracle as O
-from oracle.ref_shim import load_reference_v1, load_reference_v2, reference_available
+from oracle import make_golden as G
 from tests.conftest import load_golden
 
 ATT = load_golden("attention")
 GCN = load_golden("gcn")
 MODEL = load_golden("model")
 V2 = load_golden("v2")
+RANDOM = load_golden("random_shapes")
+PORT = load_golden("timing_port")
+
+
+def _same_inputs(case, **tensors):
+    """The inputs regenerated from their seeds are the ones the reference ran on (fp64 sums recorded with its outputs)."""
+    for name, t in tensors.items():
+        want = case["sum_" + name]
+        assert abs(float(t.double().sum()) - want) <= 1e-9 * max(1.0, abs(want)), f"input {name} differs from the recorded one"
 
 
 def _attn(name, c, dtype):
@@ -101,50 +110,56 @@ def test_v2_model_forward():
     assert O.rel_err(out, c["out"]) < 2e-5
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present (GPU box)")
 def test_oracle_against_live_reference_random_shapes():
-    ref, ref2 = load_reference_v1(), load_reference_v2()
-    gen = torch.Generator().manual_seed(0)
-    for n, h, d, hv in [(50, 1, 8, 1), (200, 4, 64, 4), (77, 3, 16, 1), (1, 2, 4, 2), (513, 2, 32, 2)]:
-        q, k, v = O.synthetic_qkv(n, h, d, seed=n, hv=hv, adversarial=True)
+    """The oracle against the reference's outputs on seeded random shapes (edge cases N = 1 and Hv = 1 < H included), recorded by
+    oracle/make_golden.py (group random_shapes) on a sample of the output rows."""
+    for n, h, d, hv, q, k, v, ei, w in G.random_shape_inputs():
+        c = RANDOM[f"shape_n{n}_h{h}_d{d}_hv{hv}"]
+        _same_inputs(c, q=q, k=k, v=v, edge_index=ei, edge_weight=w)
+        rows = c["rows"]
         # nearly-centred V amplifies fp32 summation noise; the fp64 arbiter below is tight
-        assert O.rel_err(O.simple_attention(q, k, v), ref.full_attention_conv(q, k, v, "simple")) < 2e-4
-        assert O.rel_err(O.sigmoid_attention(q * .2, k * .2, v), ref.full_attention_conv(q * .2, k * .2, v, "sigmoid")) < 1e-5
-        ei = torch.randint(0, n, (2, 5 * n), generator=gen)
-        w = torch.rand(5 * n, generator=gen)
-        assert O.rel_err(O.gcn_conv(v, ei, w), ref.gcn_conv(v, ei, w)) < 1e-5
+        assert O.rel_err(O.simple_attention(q, k, v)[rows], c["simple"]) < 2e-4
+        assert O.rel_err(O.sigmoid_attention(q * .2, k * .2, v)[rows], c["sigmoid"]) < 1e-5
+        assert O.rel_err(O.gcn_conv(v, ei, w)[rows], c["gcn"]) < 1e-5
         # fp64 arbiter
-        qd, kd, vd = q.double(), k.double(), v.double()
-        torch.set_default_dtype(torch.float64)      # the reference builds its `ones` in the default dtype
-        try:
-            want = ref.full_attention_conv(qd, kd, vd, "simple")
-        finally:
-            torch.set_default_dtype(torch.float32)
-        assert O.rel_err(O.simple_attention(qd, kd, vd), want) < 1e-12
-    nn_ = torch.tensor([3, 10, 1, 25])
-    q, k, v = O.synthetic_qkv(39, 1, 16, seed=4)
-    assert O.rel_err(O.segmented_simple_attention(q, k, v, nn_),
-                     ref2.TransConv(16, 16).full_attention(q, k, v, "simple", nn_)) < 1e-5
+        assert O.rel_err(O.simple_attention(q.double(), k.double(), v.double())[rows], c["simple64"]) < 1e-12
+    c = RANDOM["segmented"]
+    q, k, v, nn_ = G.segmented_inputs()
+    _same_inputs(c, q=q, k=k, v=v)
+    assert torch.equal(nn_, c["n_nodes"])
+    assert O.rel_err(O.segmented_simple_attention(q, k, v, nn_), c["out"]) < 1e-5
 
 
-@pytest.mark.skipif(not reference_available(), reason="no reference tree (neither /root/reference nor oracle/_ref)")
 def test_timing_port_is_bit_equal_to_the_reference_function():
     """`bench.py`'s CPU baseline times the real `full_attention_conv` when oracle/_ref exists and this port of it otherwise:
-    the port must compute exactly the reference's values (same op chain, fp32)."""
-    ref = load_reference_v1()
-    for n, h, d in [(300, 4, 64), (129, 1, 32)]:
+    the port must compute exactly the reference's values.  It runs the reference's op chain -- the same aten ops on the same
+    shapes and dtypes, in the same order, hence the same values bit for bit on any one machine -- and its output matches the
+    reference's recorded output to fp32 reassociation noise (the recording machine's thread count and vector ISA set the last bits)."""
+    for n, h, d in G.TIMING_PORT_SHAPES:
+        c = PORT[f"n{n}_h{h}_d{d}"]
         q, k, v = O.synthetic_qkv(n, h, d, seed=n)
-        assert torch.equal(O.simple_attention_reference_chain(q, k, v), ref.full_attention_conv(q, k, v, "simple"))
+        _same_inputs(c, q=q, k=k, v=v)
+        assert G.op_chain(O.simple_attention_reference_chain, q, k, v) == json.loads(c["op_chain"])
+        assert O.rel_err(O.simple_attention_reference_chain(q, k, v)[c["rows"]], c["out"]) < 1e-5
 
 
-def test_vendored_reference_is_a_byte_copy():
-    """oracle/_ref (git-ignored build output of oracle/build_ref.py) must be the unmodified files."""
-    import filecmp
+def test_vendored_reference_is_a_byte_copy(tmp_path, monkeypatch):
+    """oracle/build_ref.py (which fills the git-ignored oracle/_ref) must copy the reference files unmodified, and keep an earlier
+    copy when the reference tree is absent.  Checked on a stand-in tree of the same layout."""
     from oracle import build_ref as B
-    if not os.path.isfile(os.path.join(B.SRC, B.FILES[0])) or not os.path.isdir(B.DST):
-        pytest.skip("needs both /root/reference and oracle/_ref")
+    src, dst = tmp_path / "src", tmp_path / "dst"
+    for i, rel in enumerate(B.FILES):
+        (src / rel).parent.mkdir(parents=True, exist_ok=True)
+        (src / rel).write_bytes(bytes(range(256)) * (i + 3) + b"\r\n\x00 trailing bytes without a newline")
+    monkeypatch.setattr(B, "SRC", str(src))
+    monkeypatch.setattr(B, "DST", str(dst))
+    assert B.build_ref(verbose=False)
     for rel in B.FILES:
-        assert filecmp.cmp(os.path.join(B.SRC, rel), os.path.join(B.DST, rel), shallow=False)
+        assert filecmp.cmp(str(src / rel), str(dst / rel), shallow=False)
+    monkeypatch.setattr(B, "SRC", str(tmp_path / "absent"))
+    assert not B.build_ref(verbose=False)
+    for rel in B.FILES:
+        assert filecmp.cmp(str(src / rel), str(dst / rel), shallow=False)
 
 
 def test_v2_sigmoid_oracle_matches_reference_golden():
