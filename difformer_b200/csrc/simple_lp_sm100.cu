@@ -69,7 +69,7 @@ __device__ __forceinline__ uint32_t make_idesc_fmt(int M, int N, int a_mn, int b
 struct LpArgs {
     ReduceArgs1 r;            // q/k/v pointers unused (tensor maps); N, rows_per_cta, ws, flags, epoch, partials, prepared, sh, n_total, dbg
     unsigned long long* flags2;
-    int store_hint, reverse, l2_hints, pf_tiles;
+    int store_hint, reverse, l2_hints;
 };
 
 // W ("wide"): ONE head of M = D = 128 on the H = 2 geometry (see PLay, simple_tc.cuh): the two 64-column halves of a row play the
@@ -315,9 +315,7 @@ __global__ void __launch_bounds__(kLpThreads, 1) simple_lp_kernel(const __grid_c
                 rec[P::offSq + 1] = sk;
             }
             if (H == 1) bar_sync_named(2, 128);
-            const int64_t pf_rows = min((int64_t)min(la.pf_tiles, my_tiles) * kTile2, r1 - r0);
-            fused_tail<H, W>(a, la.flags2, rec, te, ew, lane, tmem, iters > 0, red, reinterpret_cast<const __nv_bfloat16*>(a.q) + r0 * (H * kDim),
-                          (uint32_t)(max((int64_t)0, pf_rows) * H * kDim * 2));
+            fused_tail<H, W>(a, la.flags2, rec, te, ew, lane, tmem, iters > 0, red);
             if (te == 0) {
                 mbar_expect_tx(&bbar, (uint32_t)P::kBBytes);
                 for (int i = 0; i < P::kBTiles * 2; ++i)
@@ -466,9 +464,7 @@ int simple_forward_lp(const void* q, const void* k, const void* v, int dtype, in
         a.sh.timeout_ns = comm_timeout_ns();
     }
     static const int hints = env_int("DIF_TC_P1_HINTS", 1), sth = env_int("DIF_TC_P2_STORE_HINT", 1), rev = env_int("DIF_TC_FUSED_REVERSE", 1);
-    static const int pft = env_int("DIF_TC_FUSED_PF_TILES", 0);
-    la.l2_hints = hints; la.store_hint = sth; la.reverse = rev; la.pf_tiles = pft;
-    a.q = reinterpret_cast<const float*>(q);            // only used as the base address of the L2 prefetch
+    la.l2_hints = hints; la.store_hint = sth; la.reverse = rev;
     a.dbg = dbg_buffer();
     const int fp16 = 0;
     CUtensorMap maps[4];

@@ -1232,14 +1232,18 @@ __global__ void __launch_bounds__(kThreadsTC, 1) bwd_apply_tc_kernel(const __gri
 //
 // Same pipelines as reduce_tma_kernel + apply_tc_kernel<0>, glued by the fused tail that already is a grid barrier:
 //   * no second launch, prologue, TMEM allocation or kernel-boundary drain between the passes;
-//   * the Q producers of pass 2 start streaming as soon as their converter role of pass 1 ends, i.e. WHILE the epilogue
-//     warps run the record / slice-sum / exchange tail (HBM is otherwise idle there): three shared-memory stages + two
-//     register stages of Q are in flight before the first pass-2 MMA can issue;
-//   * a CTA applies pass 2 to the rows it streamed in pass 1, last tile first: the Q rows it read most recently (L2
+//   * pass 1 is split in two phases.  Phase A streams K and V only (TMA) and yields S, z, u and sum k^2: everything the
+//     record / slice-sum / exchange / B-image tail needs.  Phase B streams Q (TMA, L2 evict_last) for sum q^2 alone, WHILE
+//     the tail warps run that tail, so HBM stays busy through the grid-wide reduction.  sum q^2 only scales the epilogue
+//     (c = 1/(|Q||K|)): it gets a grid round of its own (flags3, fused_sq_sum) that only the epilogue waits for.  With many
+//     rows per CTA (FusedArgs::split_q = 0, see kSplitQRows) phase A streams Q together with K and V and phase B is empty;
+//   * the Q producers of pass 2 start right after phase B; the MMA issuer fills the accumulator ring as soon as the B image
+//     is in shared memory;
+//   * a CTA applies pass 2 to the rows it streamed in phase B, last tile first: the Q rows it read most recently (L2
 //     evict_last) are consumed while they are still resident.
-// Warps: 0-7 converters -> Q producers; 8-11 TMA issuer (warp 8) + tail -> epilogue; 12 MMA issuer of both passes.
-// Shared memory: the two passes alias one dynamic allocation ([stg | ops] vs [Bop | Q stages | out staging | u]); the
-// slice-sum buffer of the tail lies over Bop (loaded afterwards), so the Q stages are free for the prefetch.
+// Warps: 0-7 converters -> Q phase B -> Q producers; 8-11 TMA issuer (warp 8) + tail -> epilogue; 12 MMA issuer of both passes.
+// Shared memory: the two passes alias one dynamic allocation ([stg | ops] vs [Bop | Q stages | out staging | u]).  The
+// phase-B ring lies behind Bop, so the B image may land over the phase-A staging ring while phase B still streams.
 // ------------------------------------------------------------------------------------------
 template <int H, bool W = false>
 __global__ void __launch_bounds__(kThreadsTC, 1) simple_fused_kernel(const __grid_constant__ FusedArgs fa, const __grid_constant__ CUtensorMap out_map) {
@@ -1258,6 +1262,13 @@ __global__ void __launch_bounds__(kThreadsTC, 1) simple_fused_kernel(const __gri
     float* us = reinterpret_cast<float*>(ostage + kOutStage);        // [H][64]
     __shared__ uint64_t sfull[G::kNSG], sempty[G::kNSG], ofull[G::kNO], oempty[G::kNO], done;
     __shared__ uint64_t full[kNS2], empty[kNS2], tfull[kNAcc], tempty[kNAcc], bbar;
+    // phase B: a 64 KB Q staging ring behind the B image (over the pass-2 stages, idle until phase B ends): the B image may
+    // land while phase B still streams.  64 KB in flight per SM keep HBM busy; 128 KB delay the tail's flag and slice loads
+    // behind the queued bulk copies (barrier 1 ends 10 us later) and make the step slower.
+    constexpr int kNQ = (64 << 10) / G::kStgT;
+    static_assert(P::kBBytes + kNQ * G::kStgT <= smem_fused_bytes<H, W>() - 1024, "phase-B ring must fit behind the B image");
+    uint8_t* qring = base + P::kBBytes;
+    __shared__ uint64_t qfull[kNQ], qempty[kNQ];
     __shared__ uint32_t tmem_slot;
     __shared__ float part[16];
     __shared__ __align__(16) float red[H == 1 ? 64 * 65 : 2048];    // z / u partial sums of the converters, S halves (H == 1), fp64 chains of the tail
@@ -1278,6 +1289,7 @@ __global__ void __launch_bounds__(kThreadsTC, 1) simple_fused_kernel(const __gri
         for (int s = 0; s < kNS2; ++s) { mbar_init(&full[s], 8); mbar_init(&empty[s], 1); }
         for (int s = 0; s < kNAcc; ++s) { mbar_init(&tfull[s], 1); mbar_init(&tempty[s], 4); }
         mbar_init(&bbar, 1);
+        for (int s = 0; s < kNQ; ++s) { mbar_init(&qfull[s], 1); mbar_init(&qempty[s], 8); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 12) tmem_alloc(&tmem_slot, 512);
@@ -1287,9 +1299,14 @@ __global__ void __launch_bounds__(kThreadsTC, 1) simple_fused_kernel(const __gri
     const uint32_t tmem = tmem_slot;
     pdl_wait();                                         // programmatic dependent launch: everything above overlapped the previous kernel
     DIF_STAMP(dbg, 1);
+    // flags3 epoch: same generation word as fused_tail (CTA 0 bumps it only after every CTA has published its record, i.e.
+    // after every thread here has read it)
+    const unsigned long long epoch3 =
+        a.epoch + *reinterpret_cast<volatile unsigned long long*>(a.flags + (int64_t)gridDim.x * kFlagStride) * 0x9E3779B97F4A7C15ull + 2;
+    float* rec = a.ws + (int64_t)blockIdx.x * a.ws_len;
 
     if (warp < 8) {
-        // =================== pass 1: converters (see reduce_tma_kernel) ===================
+        // =================== pass 1, phase A: converters of K and V (+ Q unless fa.split_q) (see reduce_tma_kernel) ===================
         float zacc[4] = {0.f, 0.f, 0.f, 0.f}, uacc[4] = {0.f, 0.f, 0.f, 0.f};
         float ssk = 0.f, ssq = 0.f;
         {
@@ -1305,7 +1322,7 @@ __global__ void __launch_bounds__(kThreadsTC, 1) simple_fused_kernel(const __gri
 #pragma unroll
                     for (int t = 0; t < 3; ++t) {
                         x[i][t] = make_float4(0.f, 0.f, 0.f, 0.f);
-                        if (node < nrows) x[i][t] = lds128(stg_base + s * G::kStg + t * G::kStgT + u * 16);
+                        if (node < nrows && (t < 2 || !fa.split_q)) x[i][t] = lds128(stg_base + s * G::kStg + t * G::kStgT + u * 16);
                     }
                 }
                 if (it >= G::kNO) mbar_wait(&oempty[o], ((it / G::kNO) - 1) & 1);
@@ -1338,15 +1355,65 @@ __global__ void __launch_bounds__(kThreadsTC, 1) simple_fused_kernel(const __gri
         }
         // hand the column sums to the tail warps (static shared memory: nothing of pass 2 aliases it)
         ssk = warp_sum(ssk);
-        ssq = warp_sum(ssq);
-        if (lane == 0) { part[warp] = ssk; part[8 + warp] = ssq; }
+        if (lane == 0) part[warp] = ssk;
 #pragma unroll
         for (int i = 0; i < 4; ++i) { red[tid * 4 + i] = zacc[i]; red[1024 + tid * 4 + i] = uacc[i]; }
         __threadfence_block();
         bar_arrive_named(1, 384);                      // barrier A: 256 arrivals here + the 128 tail threads' sync
-        // pass 1 still reads the staging / operand rings of the LAST stages (TMA landed, MMAs pending): the Q stages of
-        // pass 2 alias them, so the prefetch into shared memory waits for `done` (all MMAs complete); the register
-        // stages are loaded right away
+        DIF_STAMP(dbg, 11);
+        // =================== pass 1, phase B (fa.split_q): sum q^2 of the CTA's Q rows ===================
+        // The stages are the pass-1 stages of the Q rows; thread tid visits their 16-byte chunks u = tid + 256 i, stage by stage,
+        // exactly as the converters of reduce_tma_kernel do: the per-thread fma chains, the warp sums and the sum over warps are
+        // bit-identical to its.  Thread 0 issues the bulk copies (L2 evict_last: pass 2 reads the rows again) into the kNQ-stage
+        // ring once the last phase-A MMAs have released the operand ring the Q ring may overlap.
+        if (fa.split_q) {
+            const uint32_t qbase = smem_u32(qring);
+            auto issue = [&](int it) {
+                const int s = it % kNQ;
+                const int64_t row = r0 + (int64_t)it * G::kNodes;
+                const uint32_t bytes = (uint32_t)(min((int64_t)G::kNodes, r1 - row) * G::kRowB);
+                mbar_expect_tx(&qfull[s], bytes);
+                tma_load_1d_hint(qbase + s * G::kStgT, a.q + row * G::kRowF, bytes, &qfull[s], policy_evict_last());
+            };
+            if (tid == 0) {
+                mbar_wait(&done, 0);
+                for (int it = 0; it < kNQ && it < iters; ++it) issue(it);
+            }
+            __syncwarp();
+            for (int it = 0; it < iters; ++it) {
+                const int s = it % kNQ;
+                const int nrows = (int)min((int64_t)G::kNodes, r1 - (r0 + (int64_t)it * G::kNodes));
+                mbar_wait(&qfull[s], (it / kNQ) & 1);
+#pragma unroll
+                for (int i = 0; i < G::kChunksPerThread; ++i) {
+                    const int u = tid + 256 * i, node = u / G::kChunksPerRow;
+                    const float4 qq = node < nrows ? lds128(qbase + s * G::kStgT + u * 16) : make_float4(0.f, 0.f, 0.f, 0.f);
+                    ssq = fmaf(qq.x, qq.x, ssq); ssq = fmaf(qq.y, qq.y, ssq); ssq = fmaf(qq.z, qq.z, ssq); ssq = fmaf(qq.w, qq.w, ssq);
+                }
+                __syncwarp();
+                if (lane == 0) mbar_arrive(&qempty[s]);
+                if (tid == 0 && it + kNQ < iters) {
+                    mbar_wait(&qempty[s], (it / kNQ) & 1);
+                    issue(it + kNQ);
+                }
+                __syncwarp();
+            }
+        }
+        // publish sum q^2 (record + flags3).  The barrier also closes the phase-B ring: the pass-2 Q stages below alias it, so no
+        // warp may store into them while another one still reads its last Q stage.
+        ssq = warp_sum(ssq);
+        if (lane == 0) part[8 + warp] = ssq;
+        __threadfence_block();
+        bar_sync_named(3, 256);
+        if (tid == 0) {
+            float sq = 0.f;
+            for (int w = 0; w < 8; ++w) sq += part[8 + w];
+            rec[P::offSq] = sq;
+            asm volatile("st.release.gpu.global.u64 [%0], %1;" :: "l"(fa.flags3 + (int64_t)blockIdx.x * kFlagStride), "l"(epoch3) : "memory");
+        }
+        DIF_STAMP(dbg, 12);
+        // without phase B, pass 1 may still read the operand ring of the LAST stages (MMAs pending): the Q stages of pass 2 alias
+        // it, so the stores into shared memory wait for `done` (all MMAs complete); the register stages are loaded right away
         // =================== pass 2: Q producers (see apply_tc_kernel) ===================
         float buf[2][4][8];
         auto issue = [&](int sc, int j, float (&dst)[8]) {
@@ -1393,23 +1460,24 @@ __global__ void __launch_bounds__(kThreadsTC, 1) simple_fused_kernel(const __gri
     } else if (warp < 12) {
         const int te = tid - 256, ew = warp - 8;        // 128 tail / epilogue threads
         if (warp == 8 && lane == 0) {
-            // =================== pass 1: TMA issuer ===================
+            // =================== pass 1, phase A: TMA issuer (K and V; Q too unless fa.split_q) ===================
             const uint32_t stg_base = smem_u32(stg);
             const uint64_t pol_first = policy_evict_first_(), pol_last = policy_evict_last();
+            const int nt = fa.split_q ? 2 : 3;
             for (int it = 0; it < iters; ++it) {
                 const int s = it % G::kNSG;
                 if (it >= G::kNSG) mbar_wait(&sempty[s], ((it / G::kNSG) - 1) & 1);
                 const int64_t row = r0 + (int64_t)it * G::kNodes;
                 const uint32_t bytes = (uint32_t)(min((int64_t)G::kNodes, r1 - row) * G::kRowB);
-                mbar_expect_tx(&sfull[s], 3 * bytes);
+                mbar_expect_tx(&sfull[s], nt * bytes);
                 if (a.l2_hints) {
                     tma_load_1d_hint(stg_base + s * G::kStg + 0 * G::kStgT, a.k + row * G::kRowF, bytes, &sfull[s], pol_first);
                     tma_load_1d_hint(stg_base + s * G::kStg + 1 * G::kStgT, a.v + row * G::kRowF, bytes, &sfull[s], pol_first);
-                    tma_load_1d_hint(stg_base + s * G::kStg + 2 * G::kStgT, a.q + row * G::kRowF, bytes, &sfull[s], pol_last);
+                    if (nt == 3) tma_load_1d_hint(stg_base + s * G::kStg + 2 * G::kStgT, a.q + row * G::kRowF, bytes, &sfull[s], pol_last);
                 } else {
                     tma_load_1d(stg_base + s * G::kStg + 0 * G::kStgT, a.k + row * G::kRowF, bytes, &sfull[s]);
                     tma_load_1d(stg_base + s * G::kStg + 1 * G::kStgT, a.v + row * G::kRowF, bytes, &sfull[s]);
-                    tma_load_1d(stg_base + s * G::kStg + 2 * G::kStgT, a.q + row * G::kRowF, bytes, &sfull[s]);
+                    if (nt == 3) tma_load_1d(stg_base + s * G::kStg + 2 * G::kStgT, a.q + row * G::kRowF, bytes, &sfull[s]);
                 }
             }
         }
@@ -1419,7 +1487,6 @@ __global__ void __launch_bounds__(kThreadsTC, 1) simple_fused_kernel(const __gri
         tc_fence_after();
         bar_sync_named(1, 384);                          // barrier A: the converters' column sums are in `red` / `part`
         if (dbg != nullptr && te == 0) dbg[blockIdx.x * kDbgSlots + 4] = gtime();
-        float* rec = a.ws + (int64_t)blockIdx.x * a.ws_len;
         for (int col = te; col < G::kRowF; col += 128) {
             float z = 0.f, u = 0.f;
             for (int t = col >> 2; t < 256; t += G::kChunksPerRow) { z += red[t * 4 + (col & 3)]; u += red[1024 + t * 4 + (col & 3)]; }
@@ -1427,22 +1494,23 @@ __global__ void __launch_bounds__(kThreadsTC, 1) simple_fused_kernel(const __gri
             rec[P::offU + col] = u;
         }
         if (te == 0) {
-            float sk = 0.f, sq = 0.f;
-            for (int w = 0; w < 8; ++w) { sk += part[w]; sq += part[8 + w]; }
-            rec[P::offSq] = sq;
+            float sk = 0.f;
+            for (int w = 0; w < 8; ++w) sk += part[w];
             rec[P::offSq + 1] = sk;
         }
         if (H == 1) bar_sync_named(2, 128);              // `red` is re-used by the tail
-        const int64_t pf_rows = min((int64_t)min(fa.pf_tiles, my_tiles) * kTile2, r1 - r0);
-        fused_tail<H, W>(a, fa.flags2, rec, te, ew, lane, tmem, iters > 0, red, a.q + r0 * G::kRowF, (uint32_t)(max((int64_t)0, pf_rows) * G::kRowB));
+        fused_tail<H, W, true>(a, fa.flags2, rec, te, ew, lane, tmem, iters > 0, red);
         if (te == 0) {
             mbar_expect_tx(&bbar, (uint32_t)P::kBBytes);
             for (int i = 0; i < P::kBTiles * 2; ++i)
                 tma_load_1d(smem_u32(Bop) + i * kBOp, a.prepared + (size_t)i * kBOp, (uint32_t)kBOp, &bbar);
         }
         for (int i = te; i < H * kDim; i += 128) us[i] = __ldcg(a.partials + P::offU + i);
-        const float cscale = 1.f / (sqrtf(__ldcg(a.partials + P::offSq)) * sqrtf(__ldcg(a.partials + P::offSq + 1)));
-        bar_sync_named(2, 128);
+        const float sk = __ldcg(a.partials + P::offSq + 1);
+        // the MMA issuer may fill the accumulator ring meanwhile: only the scaling below waits for sum q^2
+        const float sq = fused_sq_sum<H, W>(a, fa.flags3, epoch3, te, red);     // ends with a 128-thread barrier: `us` is complete
+        if (dbg != nullptr && te == 0) dbg[blockIdx.x * kDbgSlots + 13] = gtime();
+        const float cscale = 1.f / (sqrtf(sq) * sqrtf(sk));
         // =================== pass 2: epilogue (see apply_tc_kernel) ===================
         const uint32_t obox = smem_u32(ostage) + ew * 2 * kOutBox;
         const uint64_t pol = policy_evict_first();
@@ -1794,6 +1862,11 @@ static int launch_fused(const FusedArgs& a, const CUtensorMap& map, int grid, cu
     return launch_persistent((const void*)simple_fused_kernel<H, W>, grid, kThreadsTC, (size_t)smem_fused_bytes<H, W>(), st, args);
 }
 
+// Q is streamed after K and V (phase B, overlapping the grid-wide reduction) when a CTA has at most this many rows.  The
+// reduction takes ~20 us whatever N is: at 896 rows per CTA (N = 132 534) the overlap saves 10 us of a 133 us step; at 11 136
+// rows (N = 1 632 803) it is a small share, and streaming K | V | Q together measured 55 us faster than the two phases (B200).
+constexpr int kSplitQRows = 4096;
+
 int simple_forward_tc(const float* q, const float* k, const float* v, int64_t N, int H, int Hv, int M, int D, double n_total,
                       float* partials, float* out, void* ws, int64_t ws_bytes, cudaStream_t st,
                       void* const* peer_bufs, int rank, int world, unsigned long long seq) {
@@ -1814,13 +1887,13 @@ int simple_forward_tc(const float* q, const float* k, const float* v, int64_t N,
     a.q = q; a.k = k; a.v = v; a.N = N; a.rows_per_cta = rpc;
     a.ws = (float*)ws; a.ws_len = ws_len; a.flags = (unsigned long long*)((char*)ws + fused_ws_flags_off(grid, ws_len));
     fa.flags2 = a.flags + (int64_t)(grid + 1) * kFlagStride;
+    fa.flags3 = fa.flags2 + (int64_t)grid * kFlagStride;
     a.epoch = epoch_src.fetch_add(0x632BE59BD9B4E019ull) | 1ull;
     a.partials = partials; a.prepared = (uint8_t*)ws + poff;
     a.vbar = nullptr;
     static const int hints = env_int("DIF_TC_P1_HINTS", 1), sth = env_int("DIF_TC_P2_STORE_HINT", 1), rev = env_int("DIF_TC_FUSED_REVERSE", 1);
-    static const int pft = env_int("DIF_TC_FUSED_PF_TILES", 0);
     a.l2_hints = hints;
-    fa.pf_tiles = pft;
+    fa.split_q = rpc <= kSplitQRows;
     a.n_total = (float)n_total;
     a.sh.world = 1;
     if (peer_bufs != nullptr && world > 1) {

@@ -97,8 +97,9 @@ struct FusedArgs {
     ReduceArgs1 r;            // pass 1 (+ tail, exchange) arguments; r.prepared = global scratch for the B-operand image (required)
     float* out;
     int store_hint, reverse;
-    int pf_tiles;             // Q tiles of this CTA's rows prefetched into L2 while the tail runs (HBM is idle there)
     unsigned long long* flags2;   // [grid] second grid barrier (B image complete)
+    unsigned long long* flags3;   // [grid] sum q^2 of the CTA is in its record
+    int split_q;                  // 1: pass 1 reads Q after K and V (phase B, while the tail runs); 0: together with them
 };
 template <int H, bool W = false>
 constexpr int smem_fused_bytes() {
@@ -227,15 +228,16 @@ int64_t tc_ws_len(int H) { return (SimpleLayout{H, H, kDim, kDim}.len() + 7) & ~
 // Grid-barrier flags of the one-kernel forward: one 128-byte line per CTA.  All CTAs poll all flags: with the flags packed 16 to
 // a line, ~19 000 polling threads hammer ten L2 lines and the flag STORES queue behind the polls (measured: a 5 us barrier).
 constexpr int kFlagStride = 16;      // u64 per flag slot
-// workspace: [records grid x ws_len f32][pad to 128][flags (grid + 1) lines][flags2 grid lines][B-operand image]
+// workspace: [records grid x ws_len f32][pad to 128][flags (grid + 1) lines][flags2 grid lines][flags3 grid lines][B-operand image]
 int64_t fused_ws_flags_off(int grid, int64_t ws_len) { return ((int64_t)grid * ws_len * 4 + 127) & ~(int64_t)127; }
-int64_t fused_ws_prepared_off(int grid, int64_t ws_len) { return fused_ws_flags_off(grid, ws_len) + (int64_t)(2 * grid + 1) * kFlagStride * 8; }
+int64_t fused_ws_prepared_off(int grid, int64_t ws_len) { return fused_ws_flags_off(grid, ws_len) + (int64_t)(3 * grid + 1) * kFlagStride * 8; }
 
 
 // ------------------------------------------------------------------------------------------
 // Fused tail of a one-kernel forward, executed by the 128 threads of the four tail / epilogue warps (te = 0..127,
 // ew = warp % 4 = TMEM lane quadrant).  On entry: all pass-1 MMAs have completed and z, u, sum q^2, sum k^2 of this CTA
-// are already in its record `rec`.  The function
+// are already in its record `rec`.  SQ_LATE: sum q^2 is not (it arrives later, see fused_sq_sum): that element is left out of
+// the partials and of the cross-GPU exchange.  The function
 //   1. drains the S accumulators (TMEM) into the record and publishes it (flag = epoch, release),
 //   2. waits for every CTA's record (all CTAs are resident: 1 CTA/SM, grid <= #SMs), reads "its" column slices of all
 //      records from L2 and sums them in a fixed order (fp64) -- deterministic, no float atomics,
@@ -264,10 +266,9 @@ __device__ __forceinline__ void poll_flags(const unsigned long long* flags, int 
     __threadfence();
 }
 
-template <int H, bool W = false>
+template <int H, bool W = false, bool SQ_LATE = false>
 __device__ __forceinline__ void fused_tail(const ReduceArgs1& a, unsigned long long* flags2, float* rec, int te, int ew, int lane,
-                                           uint32_t tmem, bool have_rows, float* red, const void* pf_ptr = nullptr,
-                                           uint32_t pf_bytes = 0) {
+                                           uint32_t tmem, bool have_rows, float* red) {
     using G = Geo<H>;
     using P = PLay<H, W>;
     uint64_t* dbg = a.dbg;
@@ -362,12 +363,6 @@ __device__ __forceinline__ void fused_tail(const ReduceArgs1& a, unsigned long l
             if (blockIdx.x == 0 && te == 0) *reinterpret_cast<volatile unsigned long long*>(a.flags + (int64_t)grid * kFlagStride) = gen + 1;
             waited = true;
             if (dbg != nullptr && te == 0) dbg[blockIdx.x * kDbgSlots + 8] = gtime();
-            // every CTA has finished pass 1: HBM idles until pass 2 starts -- pull the Q rows pass 2 reads LAST into L2 now
-            // (earlier would steal bandwidth from the CTAs still streaming pass 1: measured)
-            if (pf_bytes > 0 && te == 32) {
-                for (uint32_t o = 0; o < pf_bytes; o += 32768u)
-                    prefetch_l2(reinterpret_cast<const char*>(pf_ptr) + o, min(32768u, pf_bytes - o));
-            }
         }
         // Slice sum.  Four groups of 32 threads; group g walks the records r = 4i + g (the four fixed chains of the sum), lane l
         // owns the four consecutive elements 4l..4l+3 of the slice and reads them as ONE 16-byte load per record straight from
@@ -415,7 +410,7 @@ __device__ __forceinline__ void fused_tail(const ReduceArgs1& a, unsigned long l
             bar_sync_named(2, 128);
         }
         const int64_t j = j0 + te;
-        const bool live = te < slice && j < P::kP;
+        const bool live = te < slice && j < P::kP && !(SQ_LATE && j == P::offSq);
         const float local = live ? reinterpret_cast<const float*>(gsum + 3 * 128)[te] : 0.f;
         float sum = local;
         if (sharded && live) {
@@ -468,6 +463,53 @@ __device__ __forceinline__ void fused_tail(const ReduceArgs1& a, unsigned long l
     asm volatile("fence.proxy.async;" ::: "memory");
     bar_sync_named(2, 128);
     if (dbg != nullptr && te == 0) dbg[blockIdx.x * kDbgSlots + 6] = gtime();
+}
+
+// Grid-wide (and cross-GPU) sum q^2 for a fused_tail<SQ_LATE>, executed by the same 128 threads after it.  Every CTA has put its
+// sum q^2 into the offSq element of its record and set its flags3 line to `epoch3`.  Every CTA sums the records itself, in the
+// order of the slice sum of fused_tail (fp64 chains over records r = g mod 4, the records beyond the last full group of four in
+// chain 0, combined as (c0 + c1) + (c2 + c3)), so the value is bit-identical to the one the two-launch path reduces.  Multi-GPU:
+// CTA 0 pushes the local value to the peers' offSq LL words; every CTA polls them (comm_ll_sum does not consume them) and adds
+// the ranks in rank order.  CTA 0 writes the result to the partials.  Returns the sum to every calling thread.
+// `red`: shared scratch of >= 257 floats (grid <= 256).  Uses named barrier 2 (128 threads).
+template <int H, bool W = false>
+__device__ __forceinline__ float fused_sq_sum(const ReduceArgs1& a, const unsigned long long* flags3, unsigned long long epoch3, int te,
+                                              float* red) {
+    using P = PLay<H, W>;
+    const int grid = gridDim.x;
+    if (te < 32) {
+        poll_flags(flags3, grid, te, epoch3);
+        for (int r = te; r < grid; r += 32) red[r] = __ldcg(a.ws + (int64_t)r * a.ws_len + P::offSq);
+        __syncwarp();
+        const int gmain = grid & ~3;
+        double c = 0.0;
+        if (te < 4)
+            for (int r = te; r < gmain; r += 4) c += (double)red[r];
+        if (te == 0)
+            for (int r = gmain; r < grid; ++r) c += (double)red[r];
+        const double c1 = __shfl_sync(0xffffffffu, c, 1), c2 = __shfl_sync(0xffffffffu, c, 2), c3 = __shfl_sync(0xffffffffu, c, 3);
+        __syncwarp();
+        if (te == 0) {
+            const float local = (float)((c + c1) + (c2 + c3));
+            float sum = local;
+            const ShardArgs& sh = a.sh;
+            if (sh.world > 1) {
+                const int xslot = (int)(sh.seq & 1);
+                const uint32_t tag = (uint32_t)sh.seq;
+                if (blockIdx.x == 0)
+                    for (int p = 1; p < sh.world; ++p) {
+                        int r = sh.rank + p;
+                        if (r >= sh.world) r -= sh.world;
+                        comm_ll_send(comm_ll_ptr(sh.bufs[r], sh.lenpad, xslot, sh.rank) + P::offSq, local, tag);
+                    }
+                sum = comm_ll_sum(sh, xslot, P::offSq, tag, local);
+            }
+            if (blockIdx.x == 0) a.partials[P::offSq] = sum;
+            red[256] = sum;
+        }
+    }
+    bar_sync_named(2, 128);
+    return red[256];
 }
 
 }  // namespace
